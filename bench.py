@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- routing decisions/s of the EPP scheduling cycle on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload config3] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload config3] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one pass of the whole hot path (prefix-block hashing -> index lookup / global-stop match -> load scoring
 -> weighted sum -> arg-max pick [-> decider -> prefill pick]) over one batch of synthetic requests.
@@ -13,6 +13,8 @@ One "step" = one pass of the whole hot path (prefix-block hashing -> index looku
 --impl reference: times the reference's CPU algorithm (the oracle port; Go is not installable here) on all host cores.
 Multi-GPU (--gpus N under torchrun): N independent replicas, each with the full index and its own batch (weak
 scaling, no data-path collective); time = max over ranks.
+--dump-outputs DIR: after the timed steps, rank 0 writes the decisions of the last timed step as DIR/<field>.npy (see
+_dump_decisions); the inputs depend only on the arguments, so two builds can be compared file by file.
 """
 from __future__ import annotations
 
@@ -33,6 +35,7 @@ os.environ.setdefault("NCCL_DEBUG_FILE", "/dev/stderr")
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True        # the benchmark leaves the source tree as it found it (it may be read-only)
 
 METRIC = "routing decisions/sec at 4K-token prompts x 4,096 endpoints"
 UNIT = "decisions/s"
@@ -125,6 +128,22 @@ def _pinned(nbytes: int, lib):
     if rc != 0:
         raise RuntimeError("epp_host_alloc failed")
     return p, np.ctypeslib.as_array(C.cast(p, C.POINTER(C.c_uint8)), shape=(nbytes,))
+
+
+DUMP_MAX_ROWS = 1 << 19                 # 8 arrays x 8 B x 2^19 rows = 32 MiB
+
+
+def _dump_decisions(out_dir: str, dec: np.ndarray):
+    """--dump-outputs: the epp_decision records a caller of the timed path receives, one float64 array per field
+    (endpoint ids are u32 and scores f64, both exact in float64), plus request.npy, the batch row of each entry.
+    Batches above DUMP_MAX_ROWS requests are written as a fixed seeded sample of rows."""
+    rows = np.arange(dec.shape[0])
+    if rows.size > DUMP_MAX_ROWS:
+        rows = np.sort(np.random.default_rng(0).choice(rows.size, DUMP_MAX_ROWS, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "request.npy"), rows.astype(np.float64))
+    for name in dec.dtype.names:
+        np.save(os.path.join(out_dir, name + ".npy"), dec[name][rows].astype(np.float64))
 
 
 def _workload(name: str, R: int | None):
@@ -398,6 +417,8 @@ def run_gpu(args, rank, world, local_rank):
     wall = time.perf_counter() - t0
     timed_ms = eng.event_elapsed_ms()
     timed_launches = int(eng.stats()["last_kernel_launches"]) * args.steps      # kernels of one async batch x K
+    if args.dump_outputs and rank == 0:
+        _dump_decisions(args.dump_outputs, epp.decisions_from_torch(dev_dec))
     barrier()
     wall = max_over_ranks(wall)
     timed_ms = max_over_ranks(timed_ms)
@@ -588,11 +609,12 @@ def run_gpu(args, rank, world, local_rank):
         dist.destroy_process_group()
 
 
-def sharded_leg(args, rank, world, local_rank, steps, warmup):
+def sharded_leg(args, rank, world, local_rank, steps, warmup, dump_dir=None):
     """BASELINE config 5: the endpoint index sharded across the GPUs (4 096 endpoints per GPU, E = 4 096 x N), every
     rank schedules the same batch of R requests; per batch two small exchanges (presence masks, best records) over
     NVLink peer memory (default) or NCCL (--sharded-nccl).  torch.distributed must be initialised when world > 1.
-    Returns the result dict on rank 0, None elsewhere.  value = R decisions per step (the ranks decide TOGETHER)."""
+    Returns the result dict on rank 0, None elsewhere.  value = R decisions per step (the ranks decide TOGETHER).
+    dump_dir: where rank 0 writes the decisions of the last timed step (_dump_decisions)."""
     import importlib
 
     import torch
@@ -646,6 +668,8 @@ def sharded_leg(args, rank, world, local_rank, steps, warmup):
     ev1.record()
     torch.cuda.synchronize()
     wall = time.perf_counter() - t0
+    if dump_dir and rank == 0:
+        _dump_decisions(dump_dir, epp.decisions_from_torch(dec))
     barrier()
     if world > 1:
         t = torch.tensor([wall], dtype=torch.float64, device="cuda")
@@ -698,7 +722,7 @@ def run_gpu_sharded(args, rank, world, local_rank):
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     epp.build.build()
     tg.build()
-    res = sharded_leg(args, rank, world, local_rank, args.steps, args.warmup)
+    res = sharded_leg(args, rank, world, local_rank, args.steps, args.warmup, dump_dir=args.dump_outputs)
     if rank == 0:
         out = {"metric": METRIC + " (endpoint-sharded index)", "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
                "dtype": "u64 (XXH64) + f64 (scores)", "data": "synthetic"}
@@ -761,7 +785,13 @@ def main():
                          "a table far larger than L2); decisions are unchanged")
     ap.add_argument("--pitch-pad", type=int, default=0,
                     help="experiment: lay the device-resident prompts out with this many pad bytes between requests")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the decisions of the last timed step as DIR/<field>.npy (float64) to compare builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the CUDA engine decided: it needs --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

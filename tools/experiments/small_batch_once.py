@@ -1,5 +1,5 @@
-import sys, ctypes as C, numpy as np
-sys.path.insert(0, "/root/repo")
+import os, sys, ctypes as C, numpy as np
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
 import torch, epp_b200 as epp
 from epp_b200 import capi
 from tools import workload_setup as helpers, tracegen as tg
