@@ -81,12 +81,13 @@ def test_hash_golden_vectors(epp):
             assert [int(x) for x in hs[0, : nb[0]]] == want, v["name"]
 
 
-@pytest.mark.parametrize("bst", [1, 2, 3, 6, 7, 8, 16, 24, 32])
-def test_hash_ragged_vs_oracle(epp, orc, bst):
+@pytest.mark.parametrize("bst,maxb", [pytest.param(b, m, id=str(b) if m == 12 else f"{b}-cap{m}")
+                                      for m in (12, 9) for b in (1, 2, 3, 6, 7, 8, 16, 24, 32)])
+def test_hash_ragged_vs_oracle(epp, orc, bst, maxb):
     """Ragged batch (empty, shorter than a block, partial tail, truncated) for block sizes hitting every XXH64 tail
-    class: bs%32==0 (vector path), bs%32 in {24,28} (mixed stripe), tiny blocks (<32 bytes, no stripe)."""
+    class: bs%32==0 (vector path), bs%32 in {24,28} (mixed stripe), tiny blocks (<32 bytes, no stripe); even and odd
+    caps (an odd cap gives the hash rows an odd pitch)."""
     rng = random.Random(bst)
-    maxb = 12
     prompts = [b"", b"a", bytes(rng.getrandbits(8) for _ in range(bst * 4 - 1)), bytes(rng.getrandbits(8) for _ in range(bst * 4))]
     for _ in range(60):
         n = rng.randint(0, bst * 4 * (maxb + 3))
@@ -100,10 +101,18 @@ def test_hash_ragged_vs_oracle(epp, orc, bst):
             want = orc.hash_prompt(p, b"mdl", bst, maxb)
             assert nb[i] == len(want), (i, len(p))
             assert [int(x) for x in hs[i, : nb[i]]] == want, (i, len(p))
-        # (b) 16-byte aligned prompt starts with explicit offsets (vector path when bs % 32 == 0)
+        # (b) 16-byte aligned prompt starts with explicit offsets (vector path when bs % 32 == 0); the padded rows make
+        # offsets[r+1]-offsets[r] longer than the prompt, so the lengths go with them
         d2, starts = _pack_aligned(prompts)
         offs2 = np.array(starts + [starts[-1] + len(prompts[-1])], dtype=np.uint64)
-        # offsets[r+1]-offsets[r] must equal the prompt length: use per-request spans via a gather copy
+        assert any(s % 32 == 16 for s in starts)
+        lens2 = np.array([len(p) for p in prompts], dtype=np.uint64)
+        hs2, nb2 = eng.hash_prompts(d2, offsets=offs2, lengths=lens2)
+        for i, p in enumerate(prompts):
+            want = orc.hash_prompt(p, b"mdl", bst, maxb)
+            assert nb2[i] == len(want), (i, len(p))
+            assert [int(x) for x in hs2[i, : nb2[i]]] == want, (i, len(p))
+        # single prompts at offset 0 of a buffer of their own
         for i in (0, 1, 2, 3, 10, 33):
             di = np.zeros(((len(prompts[i]) + 31) // 16) * 16 + 16, np.uint8)
             di[: len(prompts[i])] = np.frombuffer(prompts[i], np.uint8)
